@@ -340,6 +340,58 @@ def oracle_dump(spec, flags, contig, pos_lo, pos_hi, lib_names):
     return o.dump(), hb, blo, (wb, ref)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, handles):
+    """--dump-outputs: the results the last timed step left in the engine handles (each handle's last window or launch), as a
+    caller of brc_fetch_device_results receives them, on a fixed seeded sample of their sites, as DIR/<name>.npy (float64;
+    the float32 statistics widened exactly).  Per sampled site: site_contig, site_pos (0-based), and per row ncover, npass,
+    pbase, flags and the 13 statistics (stats); sec_records: the secondary records (indel alleles, further base classes) of
+    the sampled sites, one per line as (site index, row, kind, indel length, read, qpos, 13 statistics), sorted."""
+    from bam_readcount_b200.engine import N_STATS, _FLOAT_STATS
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(1234)
+
+    def wide(st):
+        out = st.astype(np.float64)
+        for k in _FLOAT_STATS:
+            out[k] = st[k].view(np.float32)
+        return out
+
+    cols = {k: [] for k in ("site_contig", "site_pos", "ncover", "npass", "pbase", "flags", "stats")}
+    sec, n_done = [], 0
+    for eng, stream in handles:
+        res = eng.fetch_device_results(stream.cuda_stream)
+        per_site = res.n_rows * (4 + N_STATS) * 8
+        k = min(res.n_slots, DUMP_BYTES // 2 // len(handles) // per_site)
+        pick = np.sort(rng.choice(res.n_slots, k, replace=False))
+        contig, pos = np.zeros(res.n_slots), np.zeros(res.n_slots)
+        for g in res.regions:
+            contig[g["slot_base"]:g["slot_base"] + g["n_slots"]] = g["tid"]
+            pos[g["slot_base"]:g["slot_base"] + g["n_slots"]] = g["first_pos"] + np.arange(g["n_slots"])
+        cols["site_contig"].append(contig[pick])
+        cols["site_pos"].append(pos[pick])
+        for name in ("ncover", "npass", "pbase", "flags"):
+            cols[name].append(getattr(res, name)[:, pick].T.astype(np.float64))
+        cols["stats"].append(wide(res.pstats[:, :, pick]).transpose(2, 1, 0))
+        for i, slot in enumerate(pick.tolist()):
+            for row in range(res.n_rows):
+                j = int(res.sec_head[row, slot])
+                while j >= 0:          # the site's chain; the pool's order depends on the device's scheduling, hence the sort below
+                    sec.append(np.concatenate([[n_done + i, row, res.sec_kind[j], res.sec_len[j], res.sec_read[j], res.sec_qpos[j]],
+                                               wide(res.sec_stats[:, j])]))
+                    j = int(res.sec_next[j])
+        n_done += k
+    out = {name: np.concatenate(v) for name, v in cols.items()}
+    sec = np.array(sec, dtype=np.float64).reshape(-1, 6 + N_STATS)
+    sec = sec[np.lexsort(sec.T[::-1])]
+    room = (DUMP_BYTES - sum(a.nbytes for a in out.values())) // sec[0].nbytes if len(sec) else 0
+    out["sec_records"] = sec[:room]
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_wgs(args, cfg_name):
     import torch
     import torch.distributed as dist
@@ -500,6 +552,9 @@ def run_wgs(args, cfg_name):
     barrier()
     elapsed_ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, [(r.eng, r.stream) for r in sorted((r for r in runners if r.window is not None),
+                                                                            key=lambda r: (r.window.contig, r.window.beg))])
     gather_overflow = 0
     if world > 1:
         for r_ in runners:
@@ -941,6 +996,9 @@ def run_deep(args):
     barrier()
     elapsed_ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        last = [i % 2 for i in range(max(len(wins) - 2, 0), len(wins))]          # the handles of the last two launches, in order
+        dump_outputs(args.dump_outputs, [(engs[h], streams[h]) for h in last])
     launches = len(wins) * args.steps * (3 + engs[0].launch_count())
 
     # stage times + parity of sampled sites (untimed)
@@ -1036,6 +1094,8 @@ def main():
     ap.add_argument("--reserve-ctas", type=int, default=0, help="N > 1: CTA slots pileup_kernel leaves free for the NCCL kernels of the gather")
     ap.add_argument("--no-resident", action="store_true", help="c4: regenerate every window inside the timed loop instead of keeping windows in HBM")
     ap.add_argument("--hbm-margin-gb", type=float, default=14.0, help="HBM left free when windows are kept resident")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the results of the last step as DIR/<name>.npy")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3

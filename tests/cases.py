@@ -7,6 +7,8 @@ them, ``site_list`` (True: -l loop, False: argv regions), flags, lib_names.
 from __future__ import annotations
 
 import gzip
+import hashlib
+import json
 import os
 import sys
 
@@ -137,3 +139,14 @@ def load_golden_text(name: str) -> str:
             return fh.read().decode("latin-1")
     with open(p, "rb") as fh:
         return fh.read().decode("latin-1")
+
+
+def assert_reference_output(key: str, stdout: bytes, stderr: bytes = None) -> None:
+    """``stdout`` (and ``stderr``) equal what the reference binary printed for the test case ``key``: its exit code, line counts
+    and SHA-256 digests are stored in tests/golden/reference_outputs.json (tests/golden/make_reference_outputs.py)."""
+    with open(os.path.join(GOLDEN, "reference_outputs.json")) as fh:
+        want = json.load(fh)[key]
+    assert want["rc"] == 0, key
+    assert (stdout.count(b"\n"), hashlib.sha256(stdout).hexdigest()) == (want["stdout_lines"], want["stdout_sha256"]), key
+    if stderr is not None:
+        assert (stderr.count(b"\n"), hashlib.sha256(stderr).hexdigest()) == (want["stderr_lines"], want["stderr_sha256"]), key

@@ -10,6 +10,7 @@ import tempfile
 import numpy as np
 import pytest
 
+import bamwrite
 import cases
 from bam_readcount_b200 import bamio
 
@@ -58,16 +59,12 @@ def test_deflate_core_matches_zlib_on_every_block(tmp_path):
     exe = os.path.join(str(tmp_path), "h")
     subprocess.check_call(["g++", "-O2", "-std=c++17", "-I", os.path.join(ROOT, "bam_readcount_b200", "csrc"), "-o", exe, src, "-lz"])
     files = [os.path.join(GOLDEN, "test.bam"), os.path.join(GOLDEN, "test_bad_rg.bam")]
-    from oracle.oracle import REF_SAMTOOLS
-    if os.path.exists(REF_SAMTOOLS):
-        from bam_readcount_b200 import synth_cb
-        sp = synth_cb.Spec(seed=2, contig_len=1280 * 200)
-        info = synth_cb.write_sample_bam(sp, 0, 0, 120, str(tmp_path), REF_SAMTOOLS)
-        files.append(info["bam"])
-        for lv in ("-u", "-1"):                        # stored blocks / fast compression
-            out = os.path.join(str(tmp_path), f"x{lv}.bam")
-            subprocess.check_call([REF_SAMTOOLS, "view", lv, "-b", "-o", out, info["bam"]])
-            files.append(out)
+    from bam_readcount_b200 import synth_cb
+    sp = synth_cb.Spec(seed=2, contig_len=1280 * 200)
+    for lv in (6, 0, 1):                               # default, stored blocks, fast compression
+        d = tmp_path / f"level{lv}"
+        d.mkdir()
+        files.append(bamwrite.write_sample_bam(sp, 0, 0, 120, str(d), level=lv)["bam"])
     nblk, bad = map(int, subprocess.check_output([exe] + files).split())
     assert bad == 0 and nblk >= 20
 
@@ -92,13 +89,10 @@ def _records_of(batch, idx):
 def test_device_decoded_batch_equals_host_decoder():
     from bam_readcount_b200.engine import Engine
     jobs = [(os.path.join(GOLDEN, "test.bam"), 20, 10402000, 10406000), (os.path.join(GOLDEN, "test_bad_rg.bam"), 20, 10402984, 10402985)]
-    from oracle.oracle import REF_SAMTOOLS
-    tmp = tempfile.mkdtemp()
-    if os.path.exists(REF_SAMTOOLS):
-        from bam_readcount_b200 import synth_cb
-        sp = synth_cb.Spec(seed=6, contig_len=1280 * 2000)
-        info = synth_cb.write_sample_bam(sp, 0, 0, 1500, tmp, REF_SAMTOOLS)
-        jobs += [(info["bam"], 0, 200_000, 1_500_000), (info["bam"], 0, 0, 50_000)]
+    from bam_readcount_b200 import synth_cb
+    sp = synth_cb.Spec(seed=6, contig_len=1280 * 2000)
+    info = bamwrite.write_sample_bam(sp, 0, 0, 1500, tempfile.mkdtemp())
+    jobs += [(info["bam"], 0, 200_000, 1_500_000), (info["bam"], 0, 0, 50_000)]
     e = Engine(per_lib=True, lib_names=["a"] * 16)
     try:
         for path, tid, beg, end in jobs:
@@ -124,13 +118,9 @@ def test_device_decoded_batch_equals_host_decoder():
 def test_region_from_compressed_span_equals_region_from_host_reads(flags):
     """brc_push_bam_span (inflate + framing + kernels, reads never on the host) == brc_push_reads of the host-decoded records."""
     from bam_readcount_b200.engine import Engine
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     from bam_readcount_b200 import synth_cb
-    tmp = tempfile.mkdtemp()
     sp = synth_cb.Spec(seed=12, contig_len=1280 * 600)
-    info = synth_cb.write_sample_bam(sp, 0, 0, 600, tmp, REF_SAMTOOLS)
+    info = bamwrite.write_sample_bam(sp, 0, 0, 600, tempfile.mkdtemp())
     hdr, host = bamio.read_bam(info["bam"])
     libs = hdr.lib_names
     rg_lib = {rg: hdr.lib_of_rg(rg) for rg in hdr.rg_lb}
@@ -157,13 +147,10 @@ def test_region_from_compressed_span_equals_region_from_host_reads(flags):
 @pytest.mark.gpu
 def test_cli_device_decode_matches_host_decode(tmp_path):
     """brc-readcount with BRC_CLI_DEVICE_DECODE=1 (compressed spans -> GPU inflate/framing) prints what the host-decode path prints."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     from bam_readcount_b200 import build, synth_cb
     exe = build.build_cli()
     sp = synth_cb.Spec(seed=21, contig_len=1280 * 500)
-    info = synth_cb.write_sample_bam(sp, 0, 0, 500, str(tmp_path), REF_SAMTOOLS)
+    info = bamwrite.write_sample_bam(sp, 0, 0, 500, str(tmp_path))
     for extra in ([], ["-p", "-q", "20", "-b", "20"]):
         args = [exe, "-w", "0"] + extra + ["-f", info["fasta"], info["bam"], "chr1:5001-600000"]
         env = dict(os.environ, BRC_CLI_WINDOW="150000")

@@ -8,6 +8,7 @@ import subprocess
 import numpy as np
 import pytest
 
+import bamwrite
 import cases
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -71,20 +72,15 @@ def test_cli_reproduces_reference_goldens(tmp_path, args, bam, golden):
 
 @pytest.mark.gpu
 def test_cli_synthetic_bam_matches_oracle(tmp_path):
-    """A coordinate-sorted synthetic BAM (written with the samtools the oracle build leaves in oracle/_ref) through the
-    CLI, whole-contig region and a site list, against the CPU oracle."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
+    """A coordinate-sorted synthetic BAM (tests/bamwrite.py) through the CLI, whole-contig region and a site list, against the
+    CPU oracle."""
     from bam_readcount_b200 import synth
     exe = _cli()
     case = cases.synthetic_case(L=40000, depth=30, seed=31, regions=((0, 1001, 38000),), site_list=False)
     name, L, seq, _ = case["contigs"][0]
     d = str(tmp_path)
     synth.write_fasta(os.path.join(d, "ref.fa"), name, np.frombuffer(seq, dtype=np.uint8))
-    synth.write_sam(os.path.join(d, "s.sam"), case["batch"], [(name, L)])
-    subprocess.check_call([REF_SAMTOOLS, "view", "-b", "-o", os.path.join(d, "s.bam"), os.path.join(d, "s.sam")])
-    subprocess.check_call([REF_SAMTOOLS, "index", os.path.join(d, "s.bam")])
+    bamwrite.write_bam(os.path.join(d, "s.bam"), case["batch"], [(name, L)])
     for fl, argv in ((dict(min_mapq=20, min_bq=20), ["-q", "20", "-b", "20"]), (dict(per_lib=True, insertion_centric=True), ["-p", "-i"])):
         want, _, _ = cases.run_oracle(case, fl, site_list=False)
         p = subprocess.run([exe, "-w", "0", "-f", os.path.join(d, "ref.fa")] + argv + [os.path.join(d, "s.bam"), "chr1:1001-38000"], capture_output=True)
@@ -96,18 +92,13 @@ def test_cli_synthetic_bam_matches_oracle(tmp_path):
 def test_cli_windowed_long_region_equals_unsplit(tmp_path):
     """brc-readcount cuts long regions into windows (bounded memory); the concatenation must equal the unsplit output,
     deletions across window edges included."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     from bam_readcount_b200 import synth
     exe = _cli()
     case = cases.synthetic_case(L=30000, depth=30, seed=41, regions=((0, 1, 30000),), site_list=False)
     name, L, seq, _ = case["contigs"][0]
     d = str(tmp_path)
     synth.write_fasta(os.path.join(d, "ref.fa"), name, np.frombuffer(seq, dtype=np.uint8))
-    synth.write_sam(os.path.join(d, "s.sam"), case["batch"], [(name, L)])
-    subprocess.check_call([REF_SAMTOOLS, "view", "-b", "-o", os.path.join(d, "s.bam"), os.path.join(d, "s.sam")])
-    subprocess.check_call([REF_SAMTOOLS, "index", os.path.join(d, "s.bam")])
+    bamwrite.write_bam(os.path.join(d, "s.bam"), case["batch"], [(name, L)])
     outs = []
     for win in ("100000000", "3777"):
         p = subprocess.run([exe, "-w", "0", "-p", "-f", os.path.join(d, "ref.fa"), os.path.join(d, "s.bam"), "chr1:1-30000"],
@@ -150,13 +141,10 @@ def _site_list_regions(L, rng):
 
 
 def _make_bam(case, d):
-    from oracle.oracle import REF_SAMTOOLS
     from bam_readcount_b200 import synth
     name, L, seq, _ = case["contigs"][0]
     synth.write_fasta(os.path.join(d, "ref.fa"), name, np.frombuffer(seq, dtype=np.uint8))
-    synth.write_sam(os.path.join(d, "s.sam"), case["batch"], [(name, L)], n_libs=len(case["lib_names"]))
-    subprocess.check_call([REF_SAMTOOLS, "view", "-b", "-o", os.path.join(d, "s.bam"), os.path.join(d, "s.sam")])
-    subprocess.check_call([REF_SAMTOOLS, "index", os.path.join(d, "s.bam")])
+    bamwrite.write_bam(os.path.join(d, "s.bam"), case["batch"], [(name, L)], n_libs=len(case["lib_names"]))
     return os.path.join(d, "s.bam"), os.path.join(d, "ref.fa")
 
 
@@ -164,9 +152,6 @@ def test_cli_site_list_fetch_merging_yields_samfetch_records(tmp_path):
     """CPU (SURVEY.md §8 f-3): consecutive site-list lines share one forward pass over the BAM instead of one index seek
     each; every region must still receive exactly the records samfetch yields.  Checked against the per-region seek path
     (BRC_CLI_NO_MERGE) and against the Python decoder."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     exe = _cli()
     case = cases.synthetic_case(L=60000, depth=30, seed=77, regions=((0, 1, 60000),), site_list=True)
     bam, _ = _make_bam(case, str(tmp_path))
@@ -196,9 +181,6 @@ def test_cli_site_list_fetch_merging_yields_samfetch_records(tmp_path):
 def test_cli_dense_site_list_matches_oracle(tmp_path):
     """A few hundred site-list lines (dense, overlapping, nested, repeated, out of order) through the merged fetch, the
     engine and the emitter, against the CPU oracle run region by region like the reference's -l loop."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     exe = _cli()
     regs = _site_list_regions(60000, np.random.default_rng(5))
     case = cases.synthetic_case(L=60000, depth=30, seed=77, regions=tuple((0, s, e) for s, e in regs), site_list=True)
@@ -219,11 +201,7 @@ def test_cli_dense_site_list_matches_oracle(tmp_path):
 def test_cli_fetch_merging_two_contigs_unsorted_and_past_the_end(tmp_path):
     """CPU: the merged fetch across contig changes, lines that go backwards, duplicates, a line past the contig's last read
     and an unknown contig — record sets identical to the one-seek-per-line path and to the Python decoder."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     import dataclasses
-    from bam_readcount_b200 import synth
     from bam_readcount_b200.batch import ReadBatch
     exe = _cli()
     a = cases.synthetic_case(L=30000, depth=20, seed=3, regions=((0, 1, 30000),), site_list=True)["batch"]
@@ -231,9 +209,7 @@ def test_cli_fetch_merging_two_contigs_unsorted_and_past_the_end(tmp_path):
     b = dataclasses.replace(b, tid=np.ones_like(b.tid))
     both = ReadBatch.concat([a, b])
     d = str(tmp_path)
-    synth.write_sam(os.path.join(d, "s.sam"), both, [("chrA", 30000), ("chrB", 20000)])
-    subprocess.check_call([REF_SAMTOOLS, "view", "-b", "-o", os.path.join(d, "s.bam"), os.path.join(d, "s.sam")])
-    subprocess.check_call([REF_SAMTOOLS, "index", os.path.join(d, "s.bam")])
+    bamwrite.write_bam(os.path.join(d, "s.bam"), both, [("chrA", 30000), ("chrB", 20000)])
     lines = [("chrA", 100, 100), ("chrA", 101, 130), ("chrB", 5000, 5000), ("chrB", 5001, 5001), ("chrA", 120, 125), ("chrA", 120, 125),
              ("chrB", 19990, 25000), ("chrA", 29999, 30000), ("chrZ", 5, 6), ("chrB", 1, 1), ("chrB", 2, 2), ("chrB", 3, 400)]
     sl = tmp_path / "sites"
@@ -314,57 +290,59 @@ def test_reference_main_through_the_c_abi_on_the_cram():
         assert p.stdout.decode("latin-1") == cases.load_golden_text(golden)
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("args,bam", [
+WARNING_CASES = [
     (["-w", "3", "-l", "site_list"], "test.bam"),
     (["-w", "2", "-p", "-l", "site_list"], "test_bad_rg.bam"),
     (["-w", "5", "-i", "REGION"], "test.bam"),
     (["-w", "0", "-l", "site_list"], "test.bam"),
     (["-w", "1", "-q", "30", "-b", "25", "REGION"], "test.bam"),
-])
+]
+REGION_FORMS = [["21:10405200"], ["21:10402985-10402985", "21:10405200"], ["21:10,402,985-10,402,990"], ["21:10402985-"],
+                ["21:10402985-10402985", "21"], ["21:-5"], ["21:10402985-10402986", "21:10402987-10402990"]]
+
+
+def warning_key(args, bam):
+    return "warnings " + " ".join(args + [bam])
+
+
+def warning_argv(ref, args, bam):
+    """The command line after the program name: -f ref, the options, the BAM, then the region if any."""
+    argv = ["-f", ref]
+    regions = []
+    for a in args:
+        if a == "REGION":
+            regions = ["21:10402980-10402995"]
+        elif a == "site_list":
+            argv.append(os.path.join(GOLDEN, "site_list"))
+        else:
+            argv.append(a)
+    return argv + [os.path.join(GOLDEN, bam)] + regions
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("args,bam", WARNING_CASES)
 def test_cli_warning_lines_match_the_reference_binary(tmp_path, args, bam):
     """STDERR parity: the per-read warning lines (R:src/lib/bamrc/ReadWarnings.hpp:39-50) name the same reads, in the same order,
-    with the same "has been emitted N times" line, as the unmodified reference binary on the same command line."""
-    from oracle.oracle import REF_BIN, have_reference_binary
-    if not have_reference_binary():
-        pytest.skip("oracle/_ref not built")
+    with the same "has been emitted N times" line, as the unmodified reference binary on the same command line (its STDOUT and
+    STDERR are stored as digests in tests/golden/reference_outputs.json)."""
     exe = _cli()
     ref = _write_ref(str(tmp_path))
-    out = {}
-    for name, binary in (("ours", exe), ("ref", REF_BIN)):
-        argv = [binary, "-f", ref]
-        regions = []
-        for a in args:
-            if a == "REGION":
-                regions = ["21:10402980-10402995"]
-            elif a == "site_list":
-                argv.append(os.path.join(GOLDEN, "site_list"))
-            else:
-                argv.append(a)
-        argv.append(os.path.join(GOLDEN, bam))
-        p = subprocess.run(argv + regions, capture_output=True)
-        assert p.returncode == 0, p.stderr.decode()[-1000:]
-        out[name] = (p.stdout, p.stderr.decode("latin-1"))
-    assert out["ours"][0] == out["ref"][0]
-    assert out["ours"][1] == out["ref"][1]
+    p = subprocess.run([exe] + warning_argv(ref, args, bam), capture_output=True)
+    assert p.returncode == 0, p.stderr.decode()[-1000:]
+    cases.assert_reference_output(warning_key(args, bam), p.stdout, p.stderr)
 
 
 @pytest.mark.gpu
 def test_cli_region_forms_match_the_reference_binary(tmp_path):
     """bam_parse_region corner cases (ADVICE r1): an open end keeps the previous / default beg-end, thousands separators are
-    accepted, "chr:-N" starts at the first base — STDOUT identical to the reference binary."""
-    from oracle.oracle import REF_BIN, have_reference_binary
-    if not have_reference_binary():
-        pytest.skip("oracle/_ref not built")
+    accepted, "chr:-N" starts at the first base — STDOUT identical to the reference binary's (stored as a digest)."""
     exe = _cli()
     ref = _write_ref(str(tmp_path))
     bam = os.path.join(GOLDEN, "test.bam")
-    for regions in (["21:10405200"], ["21:10402985-10402985", "21:10405200"], ["21:10,402,985-10,402,990"], ["21:10402985-"],
-                    ["21:10402985-10402985", "21"], ["21:-5"], ["21:10402985-10402986", "21:10402987-10402990"]):
+    for regions in REGION_FORMS:
         o = subprocess.run([exe, "-w", "0", "-f", ref, bam] + regions, capture_output=True)
-        r = subprocess.run([REF_BIN, "-w", "0", "-f", ref, bam] + regions, capture_output=True)
-        assert o.returncode == r.returncode == 0
-        assert o.stdout == r.stdout, regions
+        assert o.returncode == 0
+        cases.assert_reference_output("region_forms " + " ".join(regions), o.stdout)
 
 
 def test_cli_reports_truncated_bam(tmp_path):
@@ -416,13 +394,10 @@ def test_cli_cram_config_2b_matches_reference_output():
 
 def test_cli_shards_partition_the_regions(tmp_path):
     """--shard RANK/COUNT: the ranks' units are a partition of the windowed regions, in order (decode-only, no device)."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     from bam_readcount_b200 import synth_cb
     exe = _cli()
     sp = synth_cb.Spec(seed=3, contig_len=1280 * 400)
-    info = synth_cb.write_sample_bam(sp, 0, 0, 400, str(tmp_path), REF_SAMTOOLS)
+    info = bamwrite.write_sample_bam(sp, 0, 0, 400, str(tmp_path))
     env = dict(os.environ, BRC_CLI_DECODE_ONLY="1", BRC_CLI_WINDOW="20000")
     whole = subprocess.run([exe, "-w", "0", info["bam"], "chr1:1001-400000", "chr1:420001-500000"], capture_output=True, env=env)
     assert whole.returncode == 0
@@ -438,13 +413,10 @@ def test_cli_shards_partition_the_regions(tmp_path):
 
 @pytest.mark.gpu
 def test_cli_sharded_output_concatenates_to_the_unsharded_output(tmp_path):
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     from bam_readcount_b200 import synth_cb
     exe = _cli()
     sp = synth_cb.Spec(seed=8, contig_len=1280 * 300)
-    info = synth_cb.write_sample_bam(sp, 0, 0, 300, str(tmp_path), REF_SAMTOOLS)
+    info = bamwrite.write_sample_bam(sp, 0, 0, 300, str(tmp_path))
     env = dict(os.environ, BRC_CLI_WINDOW="50000")
     args = ["-w", "0", "-i", "-f", info["fasta"], info["bam"], "chr1:2001-380000"]
     whole = subprocess.run([exe] + args, capture_output=True, env=env)
@@ -458,13 +430,10 @@ def test_cli_parallel_window_decode_yields_samfetch_records(tmp_path):
     """Big fetches are decoded by several threads over position sub-ranges (ParallelFetcher) and concatenated: record count,
     position sum and quality sum per region must equal the sequential reader's, whatever the thread count and window size
     (decode-only, no device)."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     from bam_readcount_b200 import synth_cb
     exe = _cli()
     sp = synth_cb.Spec(seed=5, contig_len=1280 * 700)
-    info = synth_cb.write_sample_bam(sp, 0, 0, 700, str(tmp_path), REF_SAMTOOLS)
+    info = bamwrite.write_sample_bam(sp, 0, 0, 700, str(tmp_path))
     regions = ["chr1:1-896000", "chr1:100001-700000", "chr1:5-300", "chr1"]
     outs = []
     for extra in ({"BRC_CLI_SEQUENTIAL": "1"}, {}, {"BRC_CLI_DECODE_THREADS": "3"}, {"BRC_CLI_DECODE_THREADS": "16", "BRC_CLI_WINDOW": "300000"},
@@ -481,9 +450,6 @@ def test_cli_parallel_window_decode_yields_samfetch_records(tmp_path):
 def test_cli_parallel_window_decode_text_and_warnings_equal_sequential(tmp_path):
     """The parallel window path (one borrowed, page-locked batch per window, next window decoded ahead) against the record-by-record
     path: STDOUT and the per-read warning lines on STDERR must be identical, also when a window boundary falls inside the region."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     from bam_readcount_b200 import synth
     from bam_readcount_b200.batch import TAG_ABSENT
     exe = _cli()
@@ -512,11 +478,7 @@ def test_cli_parallel_window_decode_two_contigs_unmapped_and_edges(tmp_path):
     """CPU: the parallel window decode on a two-contig BAM with placed-but-unmapped records, a fetch that starts inside a read,
     a fetch past the last read, a site-list line long enough to be cut into windows, and a contig without reads behind it:
     per-region (count, position sum, quality sum) identical to the sequential reader and to the Python decoder's samfetch."""
-    from oracle.oracle import REF_SAMTOOLS
-    if not os.path.exists(REF_SAMTOOLS):
-        pytest.skip("oracle/_ref/samtools not built")
     import dataclasses
-    from bam_readcount_b200 import synth
     from bam_readcount_b200.batch import ReadBatch
     exe = _cli()
     a = cases.synthetic_case(L=600000, depth=4, seed=31, regions=((0, 1, 600000),), site_list=False)["batch"]
@@ -527,9 +489,7 @@ def test_cli_parallel_window_decode_two_contigs_unmapped_and_edges(tmp_path):
     b = dataclasses.replace(b, tid=np.ones_like(b.tid))
     both = ReadBatch.concat([a, b])
     d = str(tmp_path)
-    synth.write_sam(os.path.join(d, "s.sam"), both, [("chrA", 600000), ("chrB", 400000), ("chrC", 300000)])
-    subprocess.check_call([REF_SAMTOOLS, "view", "-b", "-o", os.path.join(d, "s.bam"), os.path.join(d, "s.sam")])
-    subprocess.check_call([REF_SAMTOOLS, "index", os.path.join(d, "s.bam")])
+    bamwrite.write_bam(os.path.join(d, "s.bam"), both, [("chrA", 600000), ("chrB", 400000), ("chrC", 300000)])
     lines = [("chrA", 1, 600000), ("chrA", 100077, 500000), ("chrB", 50, 399000), ("chrA", 300000, 300001), ("chrB", 120000, 400000),
              ("chrC", 1, 300000), ("chrA", 590000, 600000)]
     sl = tmp_path / "sites"

@@ -7,7 +7,6 @@ full-width view, and a region computed window by window equals the region comput
 """
 import os
 import socket
-import tempfile
 
 import numpy as np
 import pytest
@@ -86,22 +85,29 @@ def test_deep_mode_groups_reads_per_site():
     assert np.all(np.diff(b.pos) >= 0)
 
 
-def test_generated_bam_reference_binary_equals_oracle():
-    from oracle.oracle import Oracle, REF_SAMTOOLS, have_reference_binary, run_reference_binary
-    if not have_reference_binary():
-        pytest.skip("oracle/_ref not built")
-    sp = sc.Spec(seed=1234, contig_len=1280 * 5000, n_contigs=2)
-    with tempfile.TemporaryDirectory() as wd:
-        info = sc.write_sample_bam(sp, 0, 0, 12, wd, REF_SAMTOOLS)
-        beg, end = 1280 * 2, 1280 * 9
-        for argv, flags in ((["-i"], dict(insertion_centric=True)), (["-q", "20", "-b", "20", "-p"], dict(min_mapq=20, min_bq=20, per_lib=True))):
-            out, err, rc = run_reference_binary(["-w", "0"] + argv + ["-f", info["fasta"], info["bam"], f"chr1:{beg + 1}-{end}"])
-            assert rc == 0
-            b, _ = sp.window_host(0, 0, 12)
-            o = Oracle(lib_names=[f"lib{i}" for i in range(8)], **flags)
-            o.region(b.select(b.fetch(0, beg - 1, end)), tid=0, beg=beg, end=end, contig="chr1", chrom_len=info["length"],
-                     ref_seq=sp.ref_host(0, 0, info["length"]), ref_win_beg=0, site_list_mode=False)
-            assert o.text() == out
+SAMPLE = (sc.Spec(seed=1234, contig_len=1280 * 5000, n_contigs=2), 12, 1280 * 2, 1280 * 9)     # spec, blocks, region [beg, end)
+SAMPLE_FLAGS = ((["-i"], dict(insertion_centric=True)), (["-q", "20", "-b", "20", "-p"], dict(min_mapq=20, min_bq=20, per_lib=True)))
+
+
+def test_generated_bam_reference_binary_equals_oracle(tmp_path):
+    """The SAM the generator writes is the batch it returns: byte for byte the SAM synth.write_sam makes of that batch, and the
+    reference binary's STDOUT on it (through samtools; stored as digests in tests/golden/reference_outputs.json) equals the
+    oracle on the batch."""
+    import ctypes
+    from bam_readcount_b200 import synth
+    from oracle.oracle import Oracle
+    sp, blocks, beg, end = SAMPLE
+    length = min(blocks * 1280 + 400, sp.contig_len)                 # the @SQ length write_sample_bam declares
+    b, _ = sp.window_host(0, 0, blocks)
+    gen, want = tmp_path / "gen.sam", tmp_path / "want.sam"
+    assert sc.load().brc_synth_write_sam(ctypes.byref(sp.c), 0, 0, blocks, str(gen).encode(), b"chr1", length, 4) == 0
+    synth.write_sam(str(want), b, [("chr1", length)], n_libs=8)
+    assert gen.read_bytes() == want.read_bytes()
+    for argv, flags in SAMPLE_FLAGS:
+        o = Oracle(lib_names=[f"lib{i}" for i in range(8)], **flags)
+        o.region(b.select(b.fetch(0, beg - 1, end)), tid=0, beg=beg, end=end, contig="chr1", chrom_len=length,
+                 ref_seq=sp.ref_host(0, 0, length), ref_win_beg=0, site_list_mode=False)
+        cases.assert_reference_output("synth_sample " + " ".join(argv), o.text().encode("latin-1"))
 
 
 def test_windows_and_weighted_shards_partition_the_genome():
